@@ -11,7 +11,7 @@ hot path over one resident batch:
     setk_apply_istft_pcm16 (fused beamform + iSTFT + peak normalisation + the wav
     writer's float -> PCM-16 conversion)
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 is launched by torch.distributed.run, one rank per GPU; utterances shard
 across ranks with no data-path collective ("scaling": "weak").  EVERY batch's
@@ -468,6 +468,8 @@ def gpu_arm(args):
                                                    round(hs1["throttled_ms"] - hs0["throttled_ms"], 1))}
     barrier()
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, wave, status)
     ms_mine = ev0.elapsed_time(ev1)
     ms = max_over_ranks(ms_mine)
     value = world * B * args.steps / (ms / 1000.0)
@@ -747,6 +749,28 @@ def other_configs(dev, world, rank, barrier, max_over_ranks, peak):
     return out
 
 
+DUMP_ROWS = 64     # utterances of the PCM-16 output written by --dump-outputs: 64 x 160000 x 4 B = 41 MB
+
+
+def dump_outputs(out_dir, wave, status):
+    """
+    What the last timed step returned to its caller (BeamformPipeline.run with pcm16_out=True), as
+    float32 .npy files in `out_dir`:
+      pcm16.npy   the enhanced PCM-16 samples of DUMP_ROWS utterances of the batch, picked by a fixed
+                  seed (all of them when the batch is smaller), in ascending order; (rows, n_out)
+      status.npy  the solver status of every utterance of the batch; (B,)
+    The int16 and int32 values are exact in float32.
+    """
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    B = wave.shape[0]
+    rows = np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_ROWS), replace=False))
+    pcm = wave.index_select(0, torch.from_numpy(rows).to(wave.device)).float().cpu().numpy()
+    np.save(os.path.join(out_dir, "pcm16.npy"), pcm)
+    np.save(os.path.join(out_dir, "status.npy"), status.float().cpu().numpy())
+
+
 _REAL_STDOUT = None
 
 
@@ -771,7 +795,13 @@ def main():
     ap.add_argument("--no-configs", action="store_true")
     ap.add_argument("--gather", choices=["peer", "nccl"], default="peer",
                     help="N > 1: how every batch's result reaches rank 0")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     # stdout carries ONE JSON line: everything else any library writes to file descriptor 1 (NCCL's
     # version banner comes from C) goes to stderr; emit() writes the line to the real stdout
     global _REAL_STDOUT

@@ -13,10 +13,9 @@ on the reference's default dtype path (float32 mask -> complex64 STFT), no file 
 timed region, every worker cycling through its own distinct synthetic utterances.
 
 Which code is timed (BASELINE.md section 3): the reference's OWN modules when its tree can be
-found -- $SETK_REFERENCE, then <repo>/baseline/_ref/scripts/sptk, then
-/root/reference/scripts/sptk -- imported under oracle/ref_shim.py (`kind` = "reference");
-otherwise this directory's numpy restatement of the same files (`kind` = "port"), which is
-what runs on the GPU box: the reference tree does not travel there.
+found -- $SETK_REFERENCE, then <repo>/baseline/_ref/scripts/sptk -- imported under
+oracle/ref_shim.py (`kind` = "reference"); otherwise this directory's numpy restatement of the
+same files (`kind` = "port").
 """
 import multiprocessing as mp
 import os
@@ -33,8 +32,7 @@ def reference_root():
     env = os.environ.get("SETK_REFERENCE")
     if env:
         cands += [env, os.path.join(env, "scripts", "sptk")]
-    cands += [os.path.join(ROOT, "baseline", "_ref", "scripts", "sptk"),
-              "/root/reference/scripts/sptk"]
+    cands += [os.path.join(ROOT, "baseline", "_ref", "scripts", "sptk")]
     for c in cands:
         if os.path.isdir(os.path.join(c, "libs")):
             return c

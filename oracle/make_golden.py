@@ -21,6 +21,11 @@ TEST INFRASTRUCTURE.  Writes:
   tests/golden/ref_configs.npz
       BASELINE.json configs 3 (reference CGMM mask -> GEV, 8 ch, 1024-pt) and 4
       (reference WPE -> MVDR, 6 ch) on short seeded utterances.
+  tests/golden/ref_restatement.npz
+      the reference's forward_stft and Mvdr / Gevd / Pmwf Beamformer.run on a
+      seeded 3-channel signal (complex128 path).
+  tests/golden/ref_kaldi_io.npz
+      CompressedMatrix blobs and what the reference's Kaldi reader decodes.
   tests/golden/PINNING.json
       what matched what, to how many LSB / what rel-inf.
 """
@@ -459,12 +464,70 @@ def wpd_cases(ref, report):
     np.savez_compressed(os.path.join(GOLD, "ref_wpd.npz"), **out)
 
 
+def restatement_cases(ref, report):
+    """
+    The reference's forward_stft and its Mvdr / Gevd / Pmwf(beta=0) Beamformer.run on a seeded
+    3-channel signal and a uniform random mask (complex128 observations), for the CPU test that
+    cross-checks the restatement against the reference's code.  The inputs are regenerated from
+    the same seed by the test; the outputs are stored at a seeded sample of 64 frequency bins (DC
+    and Nyquist included) to keep the fixture small: bins are independent in all of them.
+    """
+    rng = np.random.default_rng(3)
+    C, N = 3, 5000
+    x = (rng.standard_normal((C, N)) * 0.1).astype(np.float32)
+    kw = dict(frame_len=512, frame_hop=256, center=True, window="hann", transpose=False)
+    S = ref_multichannel_stft(ref, x, round_power_of_two=True, **kw)                 # c64 C x F x T
+    T, F = S.shape[2], S.shape[1]
+    mask = rng.uniform(0, 1, (T, F))
+    obs = S.astype(np.complex128)
+    bins = np.unique(np.concatenate([[0, F - 1], np.random.default_rng(4).choice(np.arange(1, F - 1), 62,
+                                                                                  replace=False)]))
+    out = {"bins": bins, "stft": S[:, bins]}
+    for kind, bf in (("mvdr", ref.beamformer.MvdrBeamformer(F)),
+                     ("gevd", ref.beamformer.GevdBeamformer(F)),
+                     ("pmwf", ref.beamformer.PmwfBeamformer(F, beta=0))):
+        out["enh_" + kind] = bf.run(mask, obs, ban=(kind == "gevd"))[bins]
+    np.savez_compressed(os.path.join(GOLD, "ref_restatement.npz"), **out)
+
+
+def kaldi_cases(ref, report):
+    """
+    The reference's Kaldi reader (libs/kaldi_io.py read_float_mat_vec) on CompressedMatrix blobs:
+    hand-built CM / CM2 / CM3 bytes (the same seeded bytes the CPU test builds) and a mask through
+    this repo's compress_kaldi_cm.  Stores each blob with what the reference decodes from it.
+    """
+    import importlib
+    import io
+    import struct
+    from setk_b200.libs.data_handler import compress_kaldi_cm
+    kio = importlib.import_module("libs.kaldi_io")
+    rng = np.random.default_rng(5)
+    rows, cols = 7, 5
+    blobs = {}
+    pch = np.sort(rng.integers(0, 65535, size=(cols, 4)), axis=1).astype("<u2")
+    u8 = rng.integers(0, 256, size=(cols, rows)).astype(np.uint8)
+    u8[0, :3] = (64, 65, 193)
+    blobs["CM"] = b"\0BCM " + struct.pack("<ffii", -3.0, 9.5, rows, cols) + pch.tobytes() + u8.tobytes()
+    u16 = rng.integers(0, 65536, size=(rows, cols)).astype("<u2")
+    blobs["CM2"] = b"\0BCM2 " + struct.pack("<ffii", 0.25, 4.0, rows, cols) + u16.tobytes()
+    u8b = rng.integers(0, 256, size=(rows, cols)).astype(np.uint8)
+    blobs["CM3"] = b"\0BCM3 " + struct.pack("<ffii", -1.0, 2.0, rows, cols) + u8b.tobytes()
+    m = (rng.random((37, 19)) ** 2).astype(np.float32)
+    blobs["mask_cm"] = b"\0BCM " + compress_kaldi_cm(m)
+    out = {}
+    for key, blob in blobs.items():
+        out[key + "/blob"] = np.frombuffer(blob, dtype=np.uint8)
+        out[key + "/ref"] = kio.read_float_mat_vec(io.BufferedReader(io.BytesIO(blob)), direct_access=True)
+    np.savez_compressed(os.path.join(GOLD, "ref_kaldi_io.npz"), **out)
+
+
 def main():
-    if len(sys.argv) > 1 and sys.argv[1] in ("cgmm", "wpe", "spatial", "fixed", "wpd"):   # add one fixture only
+    if len(sys.argv) > 1 and sys.argv[1] in ("cgmm", "wpe", "spatial", "fixed", "wpd", "restatement",
+                                             "kaldi"):   # add one fixture only
         ref = ref_shim.load_reference()
         report = {}
         {"cgmm": cgmm_cases, "wpe": wpe_cases, "spatial": spatial_cases, "fixed": fixed_cases,
-         "wpd": wpd_cases}[sys.argv[1]](ref, report)
+         "wpd": wpd_cases, "restatement": restatement_cases, "kaldi": kaldi_cases}[sys.argv[1]](ref, report)
         path = os.path.join(GOLD, "PINNING.json")
         with open(path) as f:
             full = json.load(f)
@@ -491,6 +554,8 @@ def main():
     spatial_cases(ref, report)
     fixed_cases(ref, report)
     wpd_cases(ref, report)
+    restatement_cases(ref, report)
+    kaldi_cases(ref, report)
     with open(os.path.join(GOLD, "PINNING.json"), "w") as f:
         json.dump(report, f, indent=1, sort_keys=True)
     print(json.dumps(report, indent=1, sort_keys=True))

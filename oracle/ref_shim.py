@@ -6,8 +6,7 @@ this container, unmodified, under a small compatibility shim.
 TEST INFRASTRUCTURE, BUILD-CONTAINER ONLY.  /root/reference does not exist on
 the GPU box; nothing in tests marked gpu, smoke() or bench.py calls this.
 It is used by oracle/make_golden.py (to generate tests/golden/*.npz and to
-validate the restatement) and by the CPU-only test that cross-checks the
-restatement when the reference tree is present.
+validate the restatement); the tests read only what that stored.
 
 Why a shim is needed (SURVEY.md section 0 finding 2, Appendix C):
   * librosa / soundfile are not installed -> stub modules; librosa.stft/istft

@@ -87,8 +87,11 @@ class StftPlan(object):
             max_batch=self.max_batch, max_samples=self.max_samples, reserved=0,
             window_host=self._win.ctypes.data_as(ctypes.POINTER(ctypes.c_double)))
         handle = ctypes.c_void_p()
+        # the handle belongs to the library that made it: close() must not hand it to another one
+        # bound later by use_library() (its memory may be device memory the other cannot free)
+        self._cdll = _lib.library()
         with self._device_ctx():
-            _lib.check(_lib.library().setk_plan_create(ctypes.byref(cfg), ctypes.byref(handle)))
+            _lib.check(self._cdll.setk_plan_create(ctypes.byref(cfg), ctypes.byref(handle)))
         self._h = handle
 
     # ------------------------------------------------------------------ misc
@@ -102,7 +105,7 @@ class StftPlan(object):
         if getattr(self, "_h", None):
             try:
                 with self._device_ctx():
-                    _lib.library().setk_plan_destroy(self._h)
+                    self._cdll.setk_plan_destroy(self._h)
             finally:
                 self._h = None
 
